@@ -10,9 +10,11 @@ ncclBroadcast per refresh tick (lig_comm_upload_snapshot_device).  The `strong` 
 is the same measurement with ONE R-request batch sharded over the N GPUs (north_star's C4).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload C4|C3|C2|C5] [--requests-per-gpu R]
+                    [--workload C4|C3|C2|C5] [--requests-per-gpu R] [--dump-outputs DIR]
 
-One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.
+One JSON line on stdout (rank 0).  See DESIGN.md "Measurement" for every field.  `value` times
+exactly K steps.  --dump-outputs DIR writes the picks of the last timed step as DIR/<field>.npy;
+the inputs are seeded, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -60,8 +62,11 @@ def parse_args():
     ap.add_argument("--requests-per-gpu", type=int, default=0,
                     help="override R per GPU (default: the workload's R)")
     ap.add_argument("--min-seconds", type=float, default=1.0,
-                    help="repeat the K-step timed region until this much device time has been "
-                         "spent, so the clock sampler sees the load; the median repeat is reported")
+                    help="untimed load before the K timed steps: passes over the batch ring until this "
+                         "much device time has been spent, so the clocks have settled and the clock "
+                         "sampler sees the load")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the picks of the last timed step (rank 0) as DIR/<field>.npy, float32")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: every GPU schedules R requests per step (default); strong: the "
                          "workload's R requests are sharded contiguously over the GPUs")
@@ -108,6 +113,23 @@ def committed_traffic(workload, info, steps_per_launch):
         return int(t["bytes_per_step"] * steps_per_launch), (
             f"capture has {cap.get('steps_per_launch')} steps per launch; scaled per step")
     return int(t["bytes_per_launch"]), "matches the launched kernel"
+
+
+DUMP_BYTES = 64 * 2**20
+
+
+def dump_picks(path, picks):
+    """One .npy per field of `picks`, as float32 (every pick field is an integer below 2^24, so the
+    values are exact).  Above DUMP_BYTES a fixed seeded sample of rows is written, with their row
+    numbers in row.npy (float64)."""
+    os.makedirs(path, exist_ok=True)
+    per_row = 4 * len(picks.dtype.names)
+    if len(picks) * per_row > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(len(picks), DUMP_BYTES // (per_row + 8), replace=False))
+        np.save(os.path.join(path, "row.npy"), rows.astype(np.float64))
+        picks = picks[rows]
+    for name in picks.dtype.names:
+        np.save(os.path.join(path, f"{name}.npy"), picks[name].astype(np.float32))
 
 
 class ClockSampler:
@@ -316,7 +338,9 @@ def run_reference(args, cfg, R):
     value = S * args.steps / dt
     sample = (f"{S} model requests per step drawn from the {args.workload} batch (P={P}, A={A}): the rate does not "
               f"depend on the batch size, the full R={R} per step would take {R / value:.0f} s")
-    loaded = sorted({os.path.basename(l.split()[-1]) for l in open("/proc/self/maps") if "/repo/" in l and ".so" in l})
+    root = os.path.realpath(ROOT) + os.sep
+    mapped = {l.split()[-1] for l in open("/proc/self/maps")}
+    loaded = sorted({os.path.basename(p) for p in mapped if p.startswith(root) and ".so" in p})
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
@@ -340,6 +364,8 @@ def main():
     cfg = dict(WL.CONFIGS[args.workload])
     R = args.requests_per_gpu or cfg["R"]
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs writes the GPU path's picks; --impl reference has none")
         return run_reference(args, cfg, R)
 
     import torch
@@ -426,6 +452,9 @@ def main():
         return d_in, d_out
 
     d_reqs, d_out = resident_ring(host_batches, nb)
+    # the last timed step writes here: with K > nb, ring outputs are written by several steps of the
+    # one launch, in no fixed order
+    d_last = torch.zeros(R * 8, dtype=torch.uint8, device=dev)
     torch.cuda.synchronize()         # built on torch's default stream; everything below runs on `stream`
     req_ptrs = [t.data_ptr() for t in d_reqs]
     out_ptrs = [t.data_ptr() for t in d_out]
@@ -510,10 +539,20 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
+    # each untimed pass walks the whole ring and ends on its last batch, so the timed steps, which
+    # start at batch 0, read batches the L2 no longer holds
+    _, _, _, warm_passes = time_regions(lambda r: launch_steps(0, nb, 2000 + r), nb, args.min_seconds)
+    t_rp = [req_ptrs[i % nb] for i in range(K)]
+    t_op = [out_ptrs[i % nb] for i in range(K - 1)] + [d_last.data_ptr()]
     launches0 = eng.kernel_launches
-    ms_region, ms_min, ms_max, reps = time_regions(lambda r: launch_steps(r * K, K, 1000 + r), K, args.min_seconds)
-    launches_per_region = (eng.kernel_launches - launches0) // reps
+    # a 1 ms gate: the first call of this code path can take the host longer than the default gate
+    # to enqueue, which would be timed as device idle
+    ms_region, _, _, _ = time_regions(lambda r: launch_steps(0, K, 1000, rp=t_rp, op=t_op), K, 0.0,
+                                      gate_cycles=2_000_000)
+    launches_per_region = eng.kernel_launches - launches0
     value = R_total * K / (ms_region / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_picks(args.dump_outputs, d_last.cpu().numpy().view(PICK_DTYPE))
 
     if args.timed_only:
         if rank == 0:
@@ -752,7 +791,7 @@ def main():
             "details": {
                 "l2": f"{nb} distinct resident batches ({nb * R * 24 / 2**20:.0f} MiB in+out) cycled: "
                       "inputs larger than the 126 MB L2",
-                "timed_region_repeats": reps, "region_ms_min_med_max": [ms_min, ms_region, ms_max],
+                "timed_steps": K, "untimed_passes_over_the_ring": warm_passes,
                 "snapshot": "resident (tables built at upload, once per refresh tick)",
                 "kernel": info},
             "e2e": {"value": e2e_value, "unit": UNIT,

@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -70,6 +71,48 @@ def test_gpu_arm_contract():
     assert cb["class_table_cpu"]["value"] > cb["optimised_cpu"]["value"] > cb["single_thread"]["value"]
     assert set(d["clocks"]) >= {"sm_mhz", "sm_max_mhz", "reasons"}
     assert d["streaming"]["errors"] == 0 and d["streaming"]["latency_us"]["p99"] > 0
+
+
+def test_dump_picks_samples_rows_above_the_cap(tmp_path, monkeypatch):
+    import bench
+    from llm_instance_gateway_b200.packer import PICK_DTYPE
+    picks = np.zeros(1000, dtype=PICK_DTYPE)
+    picks["pod_idx"] = np.arange(1000) - 1
+    picks["status"] = np.arange(1000) % 4
+    picks["n_survivors"] = np.arange(1000) % 65536
+    bench.dump_picks(str(tmp_path / "whole"), picks)
+    assert sorted(os.listdir(tmp_path / "whole")) == ["n_survivors.npy", "pod_idx.npy", "status.npy"]
+    for name in PICK_DTYPE.names:
+        got = np.load(tmp_path / "whole" / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, picks[name])
+    monkeypatch.setattr(bench, "DUMP_BYTES", 2000)
+    for d in ("a", "b"):
+        bench.dump_picks(str(tmp_path / d), picks)
+    rows = np.load(tmp_path / "a" / "row.npy")
+    assert rows.dtype == np.float64 and len(rows) == 2000 // 20 and np.all(np.diff(rows) > 0)
+    for name in ("row",) + PICK_DTYPE.names:                                # the sample is seeded
+        assert np.array_equal(np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "pod_idx.npy"), picks["pod_idx"][rows.astype(np.int64)])
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(tmp_path, oracle):
+    """K timed steps over a ring of the 4 host-generated batches: step K-1 reads batch (K-1) % 4 with
+    seed 1000 + K-1, and --dump-outputs writes exactly its picks."""
+    from llm_instance_gateway_b200 import workload as WL
+    K = 7
+    d = run_bench("--workload", "C3", "--steps", str(K), "--warmup", "3", "--ring", "4", "--min-seconds", "0",
+                  "--no-extras", "--no-streaming", "--no-cpu-baseline", "--dump-outputs", str(tmp_path))
+    assert d["steps"] == K and d["details"]["timed_steps"] == K
+    c = WL.CONFIGS["C3"]
+    pk = WL.make_snapshot(c["P"], c["A"]).packed
+    reqs = WL.make_requests(c["R"], c["A"], seed=WL.REQUEST_SEED + (K - 1) % 4)
+    tab = oracle.ClassTable(pk.P, pk.A, pk.kv, pk.q, pk.n_active, pk.max_active, pk.bitmap)
+    want = tab.schedule_batch(reqs, 1000 + K - 1)
+    assert sorted(os.listdir(tmp_path)) == ["n_survivors.npy", "pod_idx.npy", "status.npy"]
+    for name in want.dtype.names:
+        got = np.load(tmp_path / f"{name}.npy")
+        assert got.dtype == np.float32 and np.array_equal(got, want[name])
 
 
 @pytest.mark.gpu
